@@ -9,6 +9,7 @@ replayed as one CUDA graph exactly as the reference examples do (example_basic_u
 
   python bench.py --gpus N --steps K --warmup W          # N>1: launched by torchrun, one rank per GPU
   python bench.py --impl reference ...                   # the CPU oracle (reference restatement) on host cores
+  python bench.py ... --dump-outputs DIR                 # also writes the last timed frame's state and contacts as DIR/<name>.npy
 
 Prints ONE JSON line (see the task contract): whole-job env-steps/s, e2e (host buffers through the public API),
 roofline of the dominant kernel, cpu_baseline, clocks.
@@ -105,7 +106,11 @@ def parse_args():
                    help="CollisionPipeline(export_contacts=False): the solver reads the contact blocks, the reference-layout Contacts arrays "
                         "are not written (an RL loop that never looks at them); NOT the default, the headline keeps the export")
     p.add_argument("--gather", default="peer", choices=["peer", "nccl"], help="N > 1: end-of-frame state gather mechanism")
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write what the last timed step computed as DIR/<name>.npy, for comparing two builds")
     a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
     select_workload(a.workload)
     if a.envs is None:
         a.envs = WL["envs"]
@@ -319,6 +324,15 @@ def run_native(args):
 
     sampler = ClockSampler(local_rank) if rank == 0 else None
     total_ms, clocks = timed(step_device, args.steps, max(args.warmup, 3), sampler)
+    outputs = None
+    if args.dump_outputs and rank == 0:  # taken now: the e2e and kernel timings below keep stepping the simulation
+        if world == 1:
+            body_q, body_qd = state_0.body_q, state_0.body_qd
+        elif peer is not None:
+            body_q, body_qd = (g.reshape(-1, g.shape[-1]) for g in peer.gathered())
+        else:
+            body_q, body_qd = gathered_q, gathered_qd
+        outputs = last_step_outputs(body_q, body_qd, state_0, contacts if pipeline.export_contacts else None)
     env_steps = envs * world * SUBSTEPS * args.steps
     value = env_steps / (total_ms * 1e-3)
     frame_ms = np.asarray(timed.last_per_step)  # rank-local per-frame device times (SURVEY.md §8(d) extras)
@@ -479,16 +493,51 @@ def run_native(args):
             "comm": {"backend": "nccl" if world > 1 else None, "nranks": world, "gather": gather_mode,
                      "gather_bytes_per_rank_per_step": int(state_0.body_q.numel() * 4 + state_0.body_qd.numel() * 4) if world > 1 else 0},
         }
+        if outputs is not None:
+            write_outputs(args.dump_outputs, outputs)
         print(json.dumps(out))
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
 
 
+CONTACT_FIELDS = ("shape0", "shape1", "point0", "point1", "offset0", "offset1", "normal", "margin0", "margin1")
+DUMP_BYTES = 60 << 20  # leaves room for the .npy headers under 64 MB in all
+
+
+def last_step_outputs(body_q, body_qd, state, contacts):
+    """Host copies of what a caller of the timed frame receives: the body state (gathered over all ranks when N > 1), the joint
+    state for Featherstone (XPBD does not write it) and, when exported, the last substep's contacts of this rank.  The contacts
+    are put in (shape0, shape1, emission) order, so a build that emits the same contacts in another order compares equal."""
+    out = {"body_q": body_q, "body_qd": body_qd}
+    if WL["solver"] == "featherstone":
+        out["joint_q"], out["joint_qd"] = state.joint_q, state.joint_qd
+    out = {k: v.cpu().numpy() for k, v in out.items()}
+    if contacts is not None:
+        n = min(int(contacts.rigid_contact_count.item()), contacts.rigid_contact_max)
+        c = {k: getattr(contacts, "rigid_contact_" + k)[:n].cpu().numpy() for k in CONTACT_FIELDS}
+        order = np.lexsort((np.arange(n), c["shape1"], c["shape0"]))
+        out["contact_count"] = np.array([n])
+        out.update({"contact_" + k: v[order] for k, v in c.items()})
+    return {k: v if v.dtype == np.float32 else v.astype(np.float64) for k, v in out.items()}
+
+
+def write_outputs(directory, outputs):
+    """``DIR/<name>.npy`` for every output.  Above DUMP_BYTES in all, each array keeps the same share of its rows, chosen by a
+    fixed seed from its length alone: arrays of one length (the contact fields) keep the same rows, and two runs the same sample."""
+    total = sum(v.nbytes for v in outputs.values())
+    keep = min(1.0, DUMP_BYTES / total) if total else 1.0
+    os.makedirs(directory, exist_ok=True)
+    for name, v in outputs.items():
+        if keep < 1.0 and len(v) > 1:
+            v = v[np.sort(np.random.default_rng(0).choice(len(v), int(len(v) * keep), replace=False))]
+        np.save(os.path.join(directory, name + ".npy"), v)
+
+
 def fast_twin_measurement(args, envs):
     import subprocess
 
-    steps = max(20, min(int(args.steps), 200))
+    steps = int(args.steps)
     cmd = [sys.executable, os.path.abspath(__file__), "--fast-fp", "--steps", str(steps), "--warmup", str(max(args.warmup, 3)),
            "--workload", args.workload, "--envs", str(envs), "--no-cpu-baseline", "--no-fast-twin"]
     if args.no_export_contacts:
