@@ -103,22 +103,23 @@ NB2_DEV float contact_delta(float err, const BodyView& a, const BodyView& b, V3 
     if (denom > 0.0f) dl /= dt * denom;
     return dl * relaxation;
 }
+// `alpha_dt` is compliance / dt, passed in so that the quotient of the kernel-wide compliance is formed once per substep
 NB2_DEV float positional_correction(float err, float derr, const BodyView& a, const BodyView& b, V3 lin_a, V3 lin_b, V3 ang_a, V3 ang_b,
-                                    float compliance, float damping, float dt) {
+                                    float compliance, float damping, float dt, float alpha_dt) {
     float denom = generalized_inv_mass(a, b, lin_a, lin_b, ang_a, ang_b);
     float alpha = compliance, gamma = compliance * damping;
     float dl = -(err + alpha * 0.0f + gamma * derr);
-    if (denom + alpha > 0.0f) dl /= (dt + gamma) * denom + alpha / dt;
+    if (denom + alpha > 0.0f) dl /= (dt + gamma) * denom + alpha_dt;
     return dl;
 }
 NB2_DEV float angular_correction(float err, float derr, const BodyView& a, const BodyView& b, V3 ang_a, V3 ang_b, float compliance,
-                                 float damping, float dt) {
+                                 float damping, float dt, float alpha_dt) {
     float denom = 0.0f;
     denom += ang_inv_mass(a.rec, ang_a);
     denom += ang_inv_mass(b.rec, ang_b);
     float alpha = compliance, gamma = compliance * damping;
     float dl = -(err + alpha * 0.0f + gamma * derr);
-    if (denom + alpha > 0.0f) dl /= (dt + gamma) * denom + alpha / dt;
+    if (denom + alpha > 0.0f) dl /= (dt + gamma) * denom + alpha_dt;
     return dl;
 }
 
@@ -192,7 +193,7 @@ NB2_DEV AxisSetup load_axis_setup(const float* p) {
 }
 
 NB2_DEV bool solve_joint(const nb2_model_desc& d, const nb2_control_view& ctl, const nb2_xpbd_params& P, int j, int body0,
-                         const float* bodies, const float* jc, float dt, Deltas& out) {
+                         const float* bodies, const float* jc, float dt, float lin_alpha_dt, float ang_alpha_dt, Deltas& out) {
     // header: bits 0-3 type, bit 4 enabled, bits 8-11 / 12-15 linear / angular dof counts
     const int hdr = jc ? jc_int(jc, JC_HDR)
                        : (d.joint_type[j] | (d.joint_enabled[j] ? 16 : 0) | (d.joint_dof_dim[2 * j] << 8) | (d.joint_dof_dim[2 * j + 1] << 12));
@@ -245,11 +246,14 @@ NB2_DEV bool solve_joint(const nb2_model_desc& d, const nb2_control_view& ctl, c
             }
             V3 lp = -lc, ap = -cross(r_p, lc), ac = cross(r_c, lc);
             float derr = dot(lp, vel_p) + dot(lc, vel_c) + dot(ap, omega_p) + dot(ac, omega_c);
-            float compliance = P.joint_linear_compliance;
+            float compliance = P.joint_linear_compliance, alpha_dt = lin_alpha_dt;
             float ke = d.joint_target_ke[axis_start];
-            if (ke > 0.0f) compliance = 1.0f / ke;
+            if (ke > 0.0f) {
+                compliance = 1.0f / ke;
+                alpha_dt = compliance / dt;
+            }
             float damping = d.joint_target_kd[axis_start];
-            float dl = positional_correction(err, derr, bp, bc, lp, lc, ap, ac, compliance, damping, dt);
+            float dl = positional_correction(err, derr, bp, bc, lp, lc, ap, ac, compliance, damping, dt, alpha_dt);
             lin_dp += lp * (dl * P.joint_linear_relaxation);
             ang_dp += ap * (dl * P.joint_angular_relaxation);
             lin_dc += lc * (dl * P.joint_linear_relaxation);
@@ -274,7 +278,7 @@ NB2_DEV bool solve_joint(const nb2_model_desc& d, const nb2_control_view& ctl, c
             V3 lc = qrot(X_wp.q, V3(dim == 0 ? 1.f : 0.f, dim == 1 ? 1.f : 0.f, dim == 2 ? 1.f : 0.f));
             V3 lp = -lc, ap = -cross(r_p, lc), ac = cross(r_c, lc);
             float derr = dot(lp, vel_p) + dot(lc, vel_c) + dot(ap, omega_p) + dot(ac, omega_c);
-            float err = 0.0f, compliance = P.joint_linear_compliance, damping = 0.0f;
+            float err = 0.0f, compliance = P.joint_linear_compliance, damping = 0.0f, alpha_dt = lin_alpha_dt;
             float derr_rel = derr - s.target_vel.get(dim);
             float lo = s.lim_lo.get(dim), up = s.lim_up.get(dim);
             if (e < lo) err = e - lo;
@@ -290,9 +294,10 @@ NB2_DEV bool solve_joint(const nb2_model_desc& d, const nb2_control_view& ctl, c
                     compliance = 1.0f / kdm;
                     damping = kdm;
                 }
+                if (ks > 0.0f || kdm > 0.0f) alpha_dt = compliance / dt;
             }
             if (fabsf(err) > 1e-9f || fabsf(derr_rel) > 1e-9f) {
-                float dl = positional_correction(err, derr_rel, bp, bc, lp, lc, ap, ac, compliance, damping, dt);
+                float dl = positional_correction(err, derr_rel, bp, bc, lp, lc, ap, ac, compliance, damping, dt, alpha_dt);
                 lin_dp += lp * (dl * P.joint_linear_relaxation);
                 ang_dp += ap * (dl * P.joint_angular_relaxation);
                 lin_dc += lc * (dl * P.joint_linear_relaxation);
@@ -337,7 +342,7 @@ NB2_DEV bool solve_joint(const nb2_model_desc& d, const nb2_control_view& ctl, c
             V3 ac(quat_c.x, quat_c.y, quat_c.z);
             V3 ap = -ac;
             float derr = dot(ap, omega_p) + dot(ac, omega_c);
-            float err = 0.0f, compliance = P.joint_angular_compliance, damping = 0.0f;
+            float err = 0.0f, compliance = P.joint_angular_compliance, damping = 0.0f, alpha_dt = ang_alpha_dt;
             float derr_rel = derr - s.target_vel.get(dim) * len(ac);
             float lo = s.lim_lo.get(dim), up = s.lim_up.get(dim);
             if (e < lo) err = e - lo;
@@ -353,8 +358,9 @@ NB2_DEV bool solve_joint(const nb2_model_desc& d, const nb2_control_view& ctl, c
                     damping = kdm;
                     compliance = 1.0f / kdm;
                 }
+                if (ks > 0.0f || kdm > 0.0f) alpha_dt = compliance / dt;
             }
-            float dl = angular_correction(err, derr_rel, bp, bc, ap, ac, compliance, damping, dt) * P.joint_angular_relaxation;
+            float dl = angular_correction(err, derr_rel, bp, bc, ap, ac, compliance, damping, dt, alpha_dt) * P.joint_angular_relaxation;
             ang_dp += ap * dl;
             ang_dc += ac * dl;
         }
@@ -740,6 +746,9 @@ xpbd_step_kernel(DevModel M, nb2_xpbd_params P, nb2_state_view sin, nb2_state_vi
     // ---- Jacobi iterations ---------------------------------------------------------------------------
     const size_t T = size_t(M.slot_total);
     const float* cb = M.cb;
+    // compliance / dt of the rows that use the solver-wide compliance (limit rows, locked axes): the same for every joint, row and
+    // iteration, so divided once here instead of in every row of every iteration
+    const float lin_alpha_dt = P.joint_linear_compliance / dt, ang_alpha_dt = P.joint_angular_compliance / dt;
     for (int it = 0; it < P.iterations; ++it) {
         // CTA barriers are not needed for correctness (a warp owns its environments); they keep the CTA's warps on the same
         // stretch of code so that the instruction stream is fetched once per CTA (see the kernel comment)
@@ -903,7 +912,8 @@ xpbd_step_kernel(DevModel M, nb2_xpbd_params P, nb2_state_view sin, nb2_state_vi
             // ---- [iteration] solve_body_joints (kernels.py:1513-2044) + ordered per-body apply
             for (int j = l; j < nj; j += L) {
                 Deltas dl;
-                bool act = solve_joint(d, ctl, P, j0 + j, b0, bodies, jcache ? jcache + j * JC_SIZE : nullptr, dt, dl);
+                bool act = solve_joint(d, ctl, P, j0 + j, b0, bodies, jcache ? jcache + j * JC_SIZE : nullptr, dt, lin_alpha_dt,
+                                       ang_alpha_dt, dl);
                 if (!act) dl = Deltas();
                 store_deltas(drec + j * DR_SIZE, dl, act ? 1.0f : 0.0f);
                 if (want_jimp && act) {  // kernels.py:2043-2044
