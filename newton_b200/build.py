@@ -64,7 +64,9 @@ def build(force: bool = False, verbose: bool = False) -> str:
 
 
 def build_variant(tag: str, defines: list[str], strict: bool = True, sources=None) -> str:
-    """Experiment helper: builds ``libnewton_b200_<tag>.so`` with extra ``-D`` flags (select it with ``NB2_LIB``)."""
+    """Builds ``libnewton_b200_<tag>.so`` from the current sources, with extra nvcc flags if any (select it with ``NB2_LIB``).
+
+    Building it from another commit's checkout gives the baseline library that ``scripts/xpbd_lib_ab.sh`` compares against."""
     lib_path = os.path.join(HERE, f"libnewton_b200_{tag}.so")
     flags = NVCC_FLAGS + (STRICT_FLAGS if strict else []) + list(defines)
     procs, objs = [], []

@@ -5,7 +5,6 @@
 // per-env explicit pair lists re-ordered by the deterministic contact key (reference geometry/contact_data.py:59-87),
 // the per-body joint adjacency used for ordered (atomic-free) Jacobi accumulation, and the env-major contact blocks.
 #include <algorithm>
-#include <cstdlib>
 #include <atomic>
 #include <cstdio>
 #include <cstring>
@@ -396,16 +395,9 @@ static nb2_status build_tables(nb2_model* m, const nb2_model_desc& d) {
     dv.has_mesh_pairs = m->has_mesh_pairs ? 1 : 0;
     m->lanes_per_env =
         std::min(32, std::max(8, pow2_at_least(std::max({dv.max_env_bodies, dv.max_env_joints, std::min(dv.max_env_pairs, 32)}))));
-    {   // small batches cannot fill the GPU with warps: give each environment a full warp so its contact / pair loops need
-        // fewer rounds (measured on 512 box stacks: xpbd_step 90 -> 68 us); large batches keep the narrowest group that fits
-        int sms = 148;
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, m->device);
-        while (m->lanes_per_env < 32 && (long long)E * m->lanes_per_env / 32 < 4LL * sms) m->lanes_per_env *= 2;
-    }
-    if (const char* ov = std::getenv("NB2_LANES")) {  // tuning override: 8, 16 or 32 lanes per environment
-        const int v = std::atoi(ov);
-        if (v == 8 || v == 16 || v == 32) m->lanes_per_env = v;
-    }
+    // small batches cannot fill the GPU with warps: give each environment a full warp so its contact / pair loops need fewer
+    // rounds (measured on 512 box stacks: xpbd_step 90 -> 68 us); large batches keep the narrowest group that fits
+    while (m->lanes_per_env < 32 && (long long)E * m->lanes_per_env / 32 < 4LL * m->sm_count) m->lanes_per_env *= 2;
     return NB2_OK;
 }
 
@@ -472,16 +464,6 @@ static nb2_status upload_tables(nb2_model* m) {
     NB2_CUDA_CHECK(cudaMemset(p, 0, (size_t(dv.env_count) + 1) * sizeof(int)));
     m->allocations.push_back(p);
     dv.env_contact_offset = static_cast<int*>(p);
-    // tile chain of the fused contact export: ticket = done = 0, epoch = 1 (zeroed status words belong to epoch 0: invalid)
-    NB2_CUDA_CHECK(cudaMalloc(&p, 4 * sizeof(int)));
-    const int sync_init[4] = {0, 0, 1, 0};
-    NB2_CUDA_CHECK(cudaMemcpy(p, sync_init, sizeof(sync_init), cudaMemcpyHostToDevice));
-    m->allocations.push_back(p);
-    dv.collide_sync = static_cast<int*>(p);
-    NB2_CUDA_CHECK(cudaMalloc(&p, std::max<size_t>(size_t(dv.env_count), 1) * sizeof(unsigned long long)));
-    NB2_CUDA_CHECK(cudaMemset(p, 0, std::max<size_t>(size_t(dv.env_count), 1) * sizeof(unsigned long long)));
-    m->allocations.push_back(p);
-    dv.collide_tile_status = static_cast<unsigned long long*>(p);
     return NB2_OK;
 }
 
@@ -632,8 +614,11 @@ nb2_status nb2_model_create(const nb2_model_desc* desc, int32_t device, nb2_mode
     }
     *out = nullptr;
     DeviceGuard guard(device);
+    int sm_count = 0;
+    NB2_CUDA_CHECK(cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, device));
     nb2_model* m = new nb2_model();
     m->device = device;
+    m->sm_count = sm_count;
     nb2_status st = build_tables(m, *desc);
     if (st == NB2_OK) st = upload_tables(m);
     if (st != NB2_OK) {

@@ -18,7 +18,6 @@
 #include <cub/device/device_radix_sort.cuh>
 
 #include "nb2_gjk.cuh"
-#include <cstdlib>
 
 #include "nb2_internal.cuh"
 #include "nb2_math.cuh"
@@ -363,10 +362,11 @@ struct __align__(4) SlotRec {
     float hi[3];
 };
 
-// Write-out staging (DevModel::lane_per_contact): the narrow phase leaves a pair's candidates in the registers of ONE lane - the 4
+// Write-out staging: the narrow phase leaves a pair's candidates in the registers of ONE lane - the 4
 // contacts of a foot would be converted and stored by that lane one after the other while the group's other lanes idle.  Instead
 // every lane drops its admitted candidates (and the pair's constants) into shared memory, and the group converts / stores them one
 // lane per CONTACT: the write_contact code runs once per round instead of up to five times, and exists once in the binary.
+// Measured against the one-lane-per-pair write-out: 656.1 -> 644.4 us per 4096-quadruped frame (profiles/r2l_min_grid_ab.txt).
 struct __align__(4) StageContact {
     float center[3], normal[3], dist;
     int pair_lane;
@@ -395,32 +395,15 @@ NB2_DEV ShapeMotion ld_motion(const SlotMotionRec& r) {
 // WARPS warps per CTA (each warp = 32/L environments): the kernel is a straight line every warp walks once, so one-warp CTAs each
 // fetch the whole instruction stream cold (48 % `stall_no_inst`, profiles/r1f_collide_kernel_quadruped.txt); warps of one CTA
 // start together and share the fetches.
-// EXPORT = true also writes the reference-layout `Contacts` arrays in the same launch (the separate contact_export_kernel is gone from
-// the default path): a CTA ("tile") knows its environments' contact counts after the pair loop; the offset of its first contact in the
-// global arrays is the sum over all earlier tiles, obtained by a decoupled look-back over one status word per tile (epoch | flag |
-// count; flag 1 = the tile's own count, 2 = inclusive prefix).  Tiles take their index from a ticket counter, so a tile only ever
-// waits on tiles that started before it; the last CTA to finish re-arms ticket / done and bumps the epoch, which makes the words of
-// the previous launch (or graph replay) invalid without a memset.  Integer sums: the offsets equal a serial scan's.
-template <int L, bool CONVEX, int WARPS, bool EXPORT>
-__global__ void __launch_bounds__(32 * WARPS) collide_kernel(DevModel M, const float* __restrict__ body_q, nb2_contacts_view out) {
+template <int L, bool CONVEX, int WARPS>
+__global__ void __launch_bounds__(32 * WARPS) collide_kernel(DevModel M, const float* __restrict__ body_q) {
     constexpr int G = 32 / L;  // environments per warp
     extern __shared__ unsigned char smem_raw[];
-    __shared__ int s_tile[2];              // tile index, epoch
-    __shared__ int s_off[WARPS * G + 1];   // per-environment contact counts -> exclusive offsets inside the tile; [WARPS*G] = tile base
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int grp = lane / L;
     const int l = lane % L;
     const unsigned gmask = (L == 32) ? 0xffffffffu : (((1u << L) - 1u) << (grp * L));
-    int tile = blockIdx.x;
-    if (EXPORT) {
-        if (threadIdx.x == 0) {
-            s_tile[0] = atomicAdd(M.collide_sync + 0, 1);
-            s_tile[1] = *reinterpret_cast<volatile int*>(M.collide_sync + 2);
-        }
-        __syncthreads();
-        tile = s_tile[0];
-    }
-    const int env = (tile * WARPS + warp) * G + grp;
+    const int env = (blockIdx.x * WARPS + warp) * G + grp;
     const bool live = env < M.env_count;
     SlotRec* slots = reinterpret_cast<SlotRec*>(smem_raw) + size_t(warp * G + grp) * M.max_env_slots_shapes;
     const nb2_model_desc& d = M.d;
@@ -430,14 +413,10 @@ __global__ void __launch_bounds__(32 * WARPS) collide_kernel(DevModel M, const f
     if (CONVEX && spec_mode != 0)
         motion = reinterpret_cast<SlotMotionRec*>(reinterpret_cast<SlotRec*>(smem_raw) + size_t(WARPS * G) * M.max_env_slots_shapes) +
                  size_t(warp * G + grp) * M.max_env_slots_shapes;
-    StageContact* stage_c = nullptr;
-    StagePair* stage_p = nullptr;
-    if (M.lane_per_contact) {
-        unsigned char* sbase = smem_raw + size_t(WARPS * G) * M.max_env_slots_shapes * (sizeof(SlotRec) + (CONVEX && spec_mode != 0 ? sizeof(SlotMotionRec) : 0)) +
-                               size_t(warp * G + grp) * stage_bytes_per_group(L);
-        stage_c = reinterpret_cast<StageContact*>(sbase);
-        stage_p = reinterpret_cast<StagePair*>(sbase + size_t(L) * 5 * sizeof(StageContact));
-    }
+    unsigned char* sbase = smem_raw + size_t(WARPS * G) * M.max_env_slots_shapes * (sizeof(SlotRec) + (CONVEX && spec_mode != 0 ? sizeof(SlotMotionRec) : 0)) +
+                           size_t(warp * G + grp) * stage_bytes_per_group(L);
+    StageContact* stage_c = reinterpret_cast<StageContact*>(sbase);
+    StagePair* stage_p = reinterpret_cast<StagePair*>(sbase + size_t(L) * 5 * sizeof(StageContact));
 
     int ss = 0, nloc = 0, nslots = 0, bs = 0, ps = 0, np = 0, slot0 = 0;
     if (live) {
@@ -658,106 +637,60 @@ __global__ void __launch_bounds__(32 * WARPS) collide_kernel(DevModel M, const f
                 if (l >= o) incl += v;
             }
             const int total = __shfl_sync(0xffffffffu, incl, L - 1, L);
-            int slot = slot0 + n_total + (incl - cnt);
-            if (stage_c) {
-                if (cnt > 0) {
-                    StagePair& sp = stage_p[l];
-                    sp.sa = sa; sp.sb = sb;
-                    sp.reff_a = reff_a; sp.reff_b = reff_b; sp.marg_a = marg_a; sp.marg_b = marg_b;
-                    int k = incl - cnt;
-    #pragma unroll
-                    for (int i = 0; i < 5; ++i) {
-                        if (!(vmask & (1u << i))) continue;
-                        StageContact& sc = stage_c[k++];
-                        st3(sc.center, cpos[i]);
-                        st3(sc.normal, cnorm[i]);
-                        sc.dist = cdist[i];
-                        sc.pair_lane = l;
-                    }
-                }
-                __syncwarp();
-                float* cb = M.cb;
-                const size_t T = size_t(M.slot_total);
-                for (int c = l; c < total; c += L) {
-                    const StageContact& sc = stage_c[c];
-                    const StagePair& sp = stage_p[sc.pair_lane];
-                    const int psa = sp.sa, psb = sp.sb;
-                    const float ra = sp.reff_a, rb = sp.reff_b;
-                    const int body0 = d.shape_body[psa], body1 = d.shape_body[psb];
-                    const Xf Xbw_a = body0 == -1 ? Xf() : xinv(ldx(body_q + 7 * body0));
-                    const Xf Xbw_b = body1 == -1 ? Xf() : xinv(ldx(body_q + 7 * body1));
-                    const int o = slot0 + n_total + c;
-                    // write_contact (collide.py:210-254): world contact -> body-frame points / offsets
-                    const V3 n = unit(ld3(sc.normal)), center = ld3(sc.center);
-                    const V3 a_w = center - n * (0.5f * sc.dist + ra);
-                    const V3 b_w = center + n * (0.5f * sc.dist + rb);
-                    const float om_a = ra + sp.marg_a, om_b = rb + sp.marg_b;
-                    const V3 p0 = xpoint(Xbw_a, a_w), p1 = xpoint(Xbw_b, b_w);
-                    const V3 o0 = xvec(Xbw_a, om_a * n), o1 = xvec(Xbw_b, -om_b * n);
-                    cb[CF_BODY_A * T + o] = __int_as_float(body0 >= 0 ? body0 - bs : -1);
-                    cb[CF_BODY_B * T + o] = __int_as_float(body1 >= 0 ? body1 - bs : -1);
-                    cb[CF_SHAPE0 * T + o] = __int_as_float(psa);
-                    cb[CF_SHAPE1 * T + o] = __int_as_float(psb);
-                    cb[CF_P0X * T + o] = p0.x; cb[CF_P0Y * T + o] = p0.y; cb[CF_P0Z * T + o] = p0.z;
-                    cb[CF_P1X * T + o] = p1.x; cb[CF_P1Y * T + o] = p1.y; cb[CF_P1Z * T + o] = p1.z;
-                    cb[CF_O0X * T + o] = o0.x; cb[CF_O0Y * T + o] = o0.y; cb[CF_O0Z * T + o] = o0.z;
-                    cb[CF_O1X * T + o] = o1.x; cb[CF_O1Y * T + o] = o1.y; cb[CF_O1Z * T + o] = o1.z;
-                    cb[CF_NX * T + o] = n.x; cb[CF_NY * T + o] = n.y; cb[CF_NZ * T + o] = n.z;
-                    cb[CF_MARGIN0 * T + o] = om_a;
-                    cb[CF_MARGIN1 * T + o] = om_b;
-                    cb[CF_MU * T + o] = (d.shape_material_mu[psa] + d.shape_material_mu[psb]) / 2.0f;
-                    cb[CF_MU_TORSIONAL * T + o] = (d.shape_material_mu_torsional[psa] + d.shape_material_mu_torsional[psb]) / 2.0f;
-                    cb[CF_MU_ROLLING * T + o] = (d.shape_material_mu_rolling[psa] + d.shape_material_mu_rolling[psb]) / 2.0f;
-                    cb[CF_KE * T + o] = 0.5f * (d.shape_material_ke[psa] + d.shape_material_ke[psb]);
-                    cb[CF_KD * T + o] = 0.5f * (d.shape_material_kd[psa] + d.shape_material_kd[psb]);
-                    cb[CF_KF * T + o] = 0.5f * (d.shape_material_kf[psa] + d.shape_material_kf[psb]);
-                    cb[CF_KA * T + o] = 0.5f * (d.shape_material_ka[psa] + d.shape_material_ka[psb]);
-                }
-                __syncwarp();  // the staging area is rewritten in the next round
-            } else if (cnt > 0) {
-                const int body0 = d.shape_body[sa], body1 = d.shape_body[sb];
-                const Xf Xbw_a = body0 == -1 ? Xf() : xinv(ldx(body_q + 7 * body0));
-                const Xf Xbw_b = body1 == -1 ? Xf() : xinv(ldx(body_q + 7 * body1));
-                const float mu = (d.shape_material_mu[sa] + d.shape_material_mu[sb]) / 2.0f;
-                const float mut = (d.shape_material_mu_torsional[sa] + d.shape_material_mu_torsional[sb]) / 2.0f;
-                const float mur = (d.shape_material_mu_rolling[sa] + d.shape_material_mu_rolling[sb]) / 2.0f;
-                const float ke = 0.5f * (d.shape_material_ke[sa] + d.shape_material_ke[sb]);
-                const float kd = 0.5f * (d.shape_material_kd[sa] + d.shape_material_kd[sb]);
-                const float kf = 0.5f * (d.shape_material_kf[sa] + d.shape_material_kf[sb]);
-                const float ka = 0.5f * (d.shape_material_ka[sa] + d.shape_material_ka[sb]);
-                float* cb = M.cb;
-                const size_t T = size_t(M.slot_total);
+            if (cnt > 0) {
+                StagePair& sp = stage_p[l];
+                sp.sa = sa; sp.sb = sb;
+                sp.reff_a = reff_a; sp.reff_b = reff_b; sp.marg_a = marg_a; sp.marg_b = marg_b;
+                int k = incl - cnt;
     #pragma unroll
                 for (int i = 0; i < 5; ++i) {
                     if (!(vmask & (1u << i))) continue;
-                    // write_contact (collide.py:210-254): world contact -> body-frame points / offsets
-                    V3 n = unit(cnorm[i]);
-                    V3 a_w = cpos[i] - n * (0.5f * cdist[i] + reff_a);
-                    V3 b_w = cpos[i] + n * (0.5f * cdist[i] + reff_b);
-                    float om_a = reff_a + marg_a, om_b = reff_b + marg_b;
-                    V3 p0 = xpoint(Xbw_a, a_w), p1 = xpoint(Xbw_b, b_w);
-                    V3 o0 = xvec(Xbw_a, om_a * n), o1 = xvec(Xbw_b, -om_b * n);
-                    cb[CF_BODY_A * T + slot] = __int_as_float(body0 >= 0 ? body0 - bs : -1);
-                    cb[CF_BODY_B * T + slot] = __int_as_float(body1 >= 0 ? body1 - bs : -1);
-                    cb[CF_SHAPE0 * T + slot] = __int_as_float(sa);
-                    cb[CF_SHAPE1 * T + slot] = __int_as_float(sb);
-                    cb[CF_P0X * T + slot] = p0.x; cb[CF_P0Y * T + slot] = p0.y; cb[CF_P0Z * T + slot] = p0.z;
-                    cb[CF_P1X * T + slot] = p1.x; cb[CF_P1Y * T + slot] = p1.y; cb[CF_P1Z * T + slot] = p1.z;
-                    cb[CF_O0X * T + slot] = o0.x; cb[CF_O0Y * T + slot] = o0.y; cb[CF_O0Z * T + slot] = o0.z;
-                    cb[CF_O1X * T + slot] = o1.x; cb[CF_O1Y * T + slot] = o1.y; cb[CF_O1Z * T + slot] = o1.z;
-                    cb[CF_NX * T + slot] = n.x; cb[CF_NY * T + slot] = n.y; cb[CF_NZ * T + slot] = n.z;
-                    cb[CF_MARGIN0 * T + slot] = om_a;
-                    cb[CF_MARGIN1 * T + slot] = om_b;
-                    cb[CF_MU * T + slot] = mu;
-                    cb[CF_MU_TORSIONAL * T + slot] = mut;
-                    cb[CF_MU_ROLLING * T + slot] = mur;
-                    cb[CF_KE * T + slot] = ke;
-                    cb[CF_KD * T + slot] = kd;
-                    cb[CF_KF * T + slot] = kf;
-                    cb[CF_KA * T + slot] = ka;
-                    slot += 1;
+                    StageContact& sc = stage_c[k++];
+                    st3(sc.center, cpos[i]);
+                    st3(sc.normal, cnorm[i]);
+                    sc.dist = cdist[i];
+                    sc.pair_lane = l;
                 }
             }
+            __syncwarp();
+            float* cb = M.cb;
+            const size_t T = size_t(M.slot_total);
+            for (int c = l; c < total; c += L) {
+                const StageContact& sc = stage_c[c];
+                const StagePair& sp = stage_p[sc.pair_lane];
+                const int psa = sp.sa, psb = sp.sb;
+                const float ra = sp.reff_a, rb = sp.reff_b;
+                const int body0 = d.shape_body[psa], body1 = d.shape_body[psb];
+                const Xf Xbw_a = body0 == -1 ? Xf() : xinv(ldx(body_q + 7 * body0));
+                const Xf Xbw_b = body1 == -1 ? Xf() : xinv(ldx(body_q + 7 * body1));
+                const int o = slot0 + n_total + c;
+                // write_contact (collide.py:210-254): world contact -> body-frame points / offsets
+                const V3 n = unit(ld3(sc.normal)), center = ld3(sc.center);
+                const V3 a_w = center - n * (0.5f * sc.dist + ra);
+                const V3 b_w = center + n * (0.5f * sc.dist + rb);
+                const float om_a = ra + sp.marg_a, om_b = rb + sp.marg_b;
+                const V3 p0 = xpoint(Xbw_a, a_w), p1 = xpoint(Xbw_b, b_w);
+                const V3 o0 = xvec(Xbw_a, om_a * n), o1 = xvec(Xbw_b, -om_b * n);
+                cb[CF_BODY_A * T + o] = __int_as_float(body0 >= 0 ? body0 - bs : -1);
+                cb[CF_BODY_B * T + o] = __int_as_float(body1 >= 0 ? body1 - bs : -1);
+                cb[CF_SHAPE0 * T + o] = __int_as_float(psa);
+                cb[CF_SHAPE1 * T + o] = __int_as_float(psb);
+                cb[CF_P0X * T + o] = p0.x; cb[CF_P0Y * T + o] = p0.y; cb[CF_P0Z * T + o] = p0.z;
+                cb[CF_P1X * T + o] = p1.x; cb[CF_P1Y * T + o] = p1.y; cb[CF_P1Z * T + o] = p1.z;
+                cb[CF_O0X * T + o] = o0.x; cb[CF_O0Y * T + o] = o0.y; cb[CF_O0Z * T + o] = o0.z;
+                cb[CF_O1X * T + o] = o1.x; cb[CF_O1Y * T + o] = o1.y; cb[CF_O1Z * T + o] = o1.z;
+                cb[CF_NX * T + o] = n.x; cb[CF_NY * T + o] = n.y; cb[CF_NZ * T + o] = n.z;
+                cb[CF_MARGIN0 * T + o] = om_a;
+                cb[CF_MARGIN1 * T + o] = om_b;
+                cb[CF_MU * T + o] = (d.shape_material_mu[psa] + d.shape_material_mu[psb]) / 2.0f;
+                cb[CF_MU_TORSIONAL * T + o] = (d.shape_material_mu_torsional[psa] + d.shape_material_mu_torsional[psb]) / 2.0f;
+                cb[CF_MU_ROLLING * T + o] = (d.shape_material_mu_rolling[psa] + d.shape_material_mu_rolling[psb]) / 2.0f;
+                cb[CF_KE * T + o] = 0.5f * (d.shape_material_ke[psa] + d.shape_material_ke[psb]);
+                cb[CF_KD * T + o] = 0.5f * (d.shape_material_kd[psa] + d.shape_material_kd[psb]);
+                cb[CF_KF * T + o] = 0.5f * (d.shape_material_kf[psa] + d.shape_material_kf[psb]);
+                cb[CF_KA * T + o] = 0.5f * (d.shape_material_ka[psa] + d.shape_material_ka[psb]);
+            }
+            __syncwarp();  // the staging area is rewritten in the next round
             n_total += total;
             if (CONVEX && seg_hi < L) {
                 // ---- mesh vs infinite plane (narrow_phase.py:1761-1861, reduce_contacts=False): the group walks the vertices L at a
@@ -775,8 +708,6 @@ __global__ void __launch_bounds__(32 * WARPS) collide_kernel(DevModel M, const f
                 const int body0 = d.shape_body[msa], body1 = d.shape_body[psb];
                 const Xf Xbw_a = body0 == -1 ? Xf() : xinv(ldx(body_q + 7 * body0));
                 const Xf Xbw_b = body1 == -1 ? Xf() : xinv(ldx(body_q + 7 * body1));
-                float* cb = M.cb;
-                const size_t T = size_t(M.slot_total);
                 int written = 0;
                 for (int v0 = 0; v0 < nv; v0 += L) {
                     const int vi = v0 + l;
@@ -831,107 +762,6 @@ __global__ void __launch_bounds__(32 * WARPS) collide_kernel(DevModel M, const f
         }
     }
     if (live && l == 0) M.env_contact_count[env] = n_total;
-    if constexpr (!EXPORT) return;
-
-    // ---- fused export: tile-local offsets, look-back for the tile base, scatter -----------------------------------------------
-    typedef unsigned long long u64;
-    constexpr int NE = WARPS * G;  // environments per tile (<= 32)
-    const unsigned epoch = unsigned(s_tile[1]) & 0x3FFFFFFFu;
-    if (l == 0) s_off[warp * G + grp] = live ? n_total : 0;
-    __syncthreads();  // also makes this CTA's contact-block stores visible to the lanes that copy them out below
-    if (warp == 0) {
-        const int mine = lane < NE ? s_off[lane] : 0;
-        int incl = mine;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const int v = __shfl_up_sync(0xffffffffu, incl, o);
-            if (lane >= o) incl += v;
-        }
-        const int tile_total = __shfl_sync(0xffffffffu, incl, 31);
-        volatile u64* status = M.collide_tile_status;
-        int base = 0;
-        if (tile > 0) {
-            if (lane == 0) status[tile] = (u64(epoch) << 34) | (1ull << 32) | u64(unsigned(tile_total));
-            // a window is 8 x 32 predecessors (word w of lane i is tile look - (32 w + i)), loaded together, so that the 256 tiles
-            // of a 4096-environment batch resolve in ONE L2 round trip - all tiles of a single-wave launch finish at about the same
-            // time, so inclusive prefixes are rarely there yet and the walk goes all the way back
-            constexpr int WORDS = 8;
-            int look = tile - 1;
-            for (;;) {
-                u64 st[WORDS];
-                for (;;) {  // spin until every predecessor of this window has published for this epoch
-                    bool valid = true;
-#pragma unroll
-                    for (int w = 0; w < WORDS; ++w) {
-                        const int idx = look - (32 * w + lane);
-                        st[w] = idx >= 0 ? status[idx] : 0ull;
-                    }
-#pragma unroll
-                    for (int w = 0; w < WORDS; ++w) {
-                        const int idx = look - (32 * w + lane);
-                        if (idx >= 0) valid = valid && unsigned(st[w] >> 34) == epoch && ((st[w] >> 32) & 3ull) != 0ull;
-                    }
-                    if (__all_sync(0xffffffffu, valid)) break;
-                }
-                bool done = false;
-#pragma unroll
-                for (int w = 0; w < WORDS; ++w) {
-                    const int idx = look - (32 * w + lane);
-                    const int flag = idx >= 0 ? int((st[w] >> 32) & 3ull) : 2, value = idx >= 0 ? int(unsigned(st[w])) : 0;
-                    const unsigned inclusive = __ballot_sync(0xffffffffu, flag == 2);
-                    const int stop = inclusive ? __ffs(inclusive) - 1 : 31;  // nearest predecessor that already holds an inclusive prefix
-                    int part = (!done && lane <= stop) ? value : 0;
-#pragma unroll
-                    for (int o = 16; o > 0; o >>= 1) part += __shfl_xor_sync(0xffffffffu, part, o);
-                    base += part;
-                    done = done || inclusive != 0u;
-                }
-                if (done) break;
-                look -= 32 * WORDS;
-            }
-        }
-        if (lane == 0) {
-            status[tile] = (u64(epoch) << 34) | (2ull << 32) | u64(unsigned(base + tile_total));
-            s_off[NE] = base;
-            if (tile == int(gridDim.x) - 1) {  // the last tile's inclusive prefix is the global count
-                M.env_contact_offset[M.env_count] = base + tile_total;
-                out.rigid_contact_count[0] = base + tile_total;
-            }
-        }
-        if (lane < NE) s_off[lane] = incl - mine;
-    }
-    __syncthreads();
-    if (live) {
-        const int dst0 = s_off[NE] + s_off[warp * G + grp];
-        if (l == 0) M.env_contact_offset[env] = dst0;
-        const size_t T = size_t(M.slot_total);
-        const float* cb = M.cb;
-        for (int c = l; c < n_total; c += L) {
-            const int s = slot0 + c, o = dst0 + c;
-            if (o >= out.rigid_contact_max) break;  // overflow: the count keeps growing, the writes are dropped (collide.py:176-177)
-            out.shape0[o] = __float_as_int(cb[CF_SHAPE0 * T + s]);
-            out.shape1[o] = __float_as_int(cb[CF_SHAPE1 * T + s]);
-#pragma unroll
-            for (int k = 0; k < 3; ++k) {
-                out.point0[3 * o + k] = cb[(CF_P0X + k) * T + s];
-                out.point1[3 * o + k] = cb[(CF_P1X + k) * T + s];
-                out.offset0[3 * o + k] = cb[(CF_O0X + k) * T + s];
-                out.offset1[3 * o + k] = cb[(CF_O1X + k) * T + s];
-                out.normal[3 * o + k] = cb[(CF_NX + k) * T + s];
-            }
-            out.margin0[o] = cb[CF_MARGIN0 * T + s];
-            out.margin1[o] = cb[CF_MARGIN1 * T + s];
-            if (out.tids) out.tids[o] = 0;
-        }
-    }
-    if (threadIdx.x == 0) {  // re-arm the chain for the next launch
-        __threadfence();
-        if (atomicAdd(M.collide_sync + 1, 1) == int(gridDim.x) - 1) {
-            M.collide_sync[0] = 0;
-            M.collide_sync[1] = 0;
-            M.collide_sync[2] = s_tile[1] + 1;
-        }
-    }
 }
 
 // ---- run-time broad phases: per-world NxN enumeration / sweep-and-prune (reference geometry/broad_phase_nxn.py:132-218,
@@ -1392,45 +1222,32 @@ nb2_status launch_contacts_import(nb2_model* m, const nb2_contacts_view& in, cud
 }
 
 template <int L, bool CONVEX, int WARPS>
-static nb2_status launch_collide_W(nb2_model* m, const float* body_q, const nb2_contacts_view* fused_out, cudaStream_t s) {
+static nb2_status launch_collide_W(nb2_model* m, const float* body_q, cudaStream_t s) {
     const DevModel& M = m->dev;
     const int NE = (32 / L) * WARPS;
     const int blocks = (M.env_count + NE - 1) / NE;
-    const size_t smem = size_t(NE) * M.max_env_slots_shapes * (sizeof(SlotRec) + (CONVEX && M.spec_mode != 0 ? sizeof(SlotMotionRec) : 0)) +
-                        (M.lane_per_contact ? size_t(NE) * stage_bytes_per_group(L) : 0);
-    if (fused_out) {
-        if (smem > 48 * 1024)
-            NB2_CUDA_CHECK(cudaFuncSetAttribute(collide_kernel<L, CONVEX, WARPS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-        collide_kernel<L, CONVEX, WARPS, true><<<blocks, 32 * WARPS, smem, s>>>(M, body_q, *fused_out);
-    } else {
-        if (smem > 48 * 1024)
-            NB2_CUDA_CHECK(cudaFuncSetAttribute(collide_kernel<L, CONVEX, WARPS, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-        collide_kernel<L, CONVEX, WARPS, false><<<blocks, 32 * WARPS, smem, s>>>(M, body_q, nb2_contacts_view{});
-    }
+    const size_t smem = size_t(NE) * (M.max_env_slots_shapes * (sizeof(SlotRec) + (CONVEX && M.spec_mode != 0 ? sizeof(SlotMotionRec) : 0)) +
+                                      stage_bytes_per_group(L));
+    if (smem > 48 * 1024)
+        NB2_CUDA_CHECK(cudaFuncSetAttribute(collide_kernel<L, CONVEX, WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+    collide_kernel<L, CONVEX, WARPS><<<blocks, 32 * WARPS, smem, s>>>(M, body_q);
     count_launch();
     NB2_CUDA_CHECK(cudaGetLastError());
     return NB2_OK;
 }
 
+// warps per CTA: 8 when the batch puts at least 8 warps on every SM, shared memory permitting
 template <int L, bool CONVEX>
-static nb2_status launch_collide_L(nb2_model* m, const float* body_q, const nb2_contacts_view* fused_out, cudaStream_t s) {
+static nb2_status launch_collide_L(nb2_model* m, const float* body_q, cudaStream_t s) {
     const DevModel& M = m->dev;
     const size_t per_warp = size_t(32 / L) * (M.max_env_slots_shapes * (sizeof(SlotRec) + (CONVEX && M.spec_mode != 0 ? sizeof(SlotMotionRec) : 0)) +
-                                              (M.lane_per_contact ? stage_bytes_per_group(L) : 0));
+                                              stage_bytes_per_group(L));
     if (per_warp > 200 * 1024) {
         set_error("collide: too many shapes per environment for the fused kernel");
         return NB2_ERR_CAPACITY;
     }
-    static const int forced = std::getenv("NB2_COLLIDE_WARPS") ? std::atoi(std::getenv("NB2_COLLIDE_WARPS")) : 0;
-    int warps = forced;
-    if (warps <= 0) {  // as many warps per CTA as the batch puts on every SM, up to 8
-        int sms = 148;
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, m->device);
-        const long long total_warps = (M.env_count + (32 / L) - 1) / (32 / L);
-        warps = (total_warps + sms - 1) / sms >= 8 ? 8 : 1;
-    }
-    if (warps >= 8 && per_warp * 8 <= 200 * 1024) return launch_collide_W<L, CONVEX, 8>(m, body_q, fused_out, s);
-    return launch_collide_W<L, CONVEX, 1>(m, body_q, fused_out, s);
+    if (warps_per_sm(m, L) >= 8 && per_warp * 8 <= 200 * 1024) return launch_collide_W<L, CONVEX, 8>(m, body_q, s);
+    return launch_collide_W<L, CONVEX, 1>(m, body_q, s);
 }
 
 template <int L>
@@ -1474,27 +1291,19 @@ nb2_status launch_collide(nb2_model* m, const float* body_q, const nb2_contacts_
         return NB2_ERR_UNSUPPORTED;
     }
     if (M.dyn_pairs && (st = launch_broadphase(m, body_q, s)) != NB2_OK) return st;
-    // NB2_COLLIDE_FUSED_EXPORT=1: the `Contacts` arrays are written by the collide kernel itself (EXPORT = true, tile chain with
-    // decoupled look-back).  Measured on B200 it LOSES to the two-kernel path (collide, then contact_export_kernel): 4096 quadruped
-    // envs, frame 690.1 vs 678.3 us L2-warm, 733.8 vs 718.0 us with L2 flushed (profiles/r2j_fused_export_ab.txt) - the 256 tiles of
-    // a single-wave launch all reach the look-back at the same time and serialise on it.  So the default is the two-kernel path.
-    static const bool fused = std::getenv("NB2_COLLIDE_FUSED_EXPORT") && std::atoi(std::getenv("NB2_COLLIDE_FUSED_EXPORT")) != 0;
-    // one lane per contact in the write-out (NB2_COLLIDE_LANE_PER_CONTACT=0: one lane per pair, the round-1 arrangement; A/B in profiles/)
-    static const bool lane_per_contact = !(std::getenv("NB2_COLLIDE_LANE_PER_CONTACT") && std::atoi(std::getenv("NB2_COLLIDE_LANE_PER_CONTACT")) == 0);
-    m->dev.lane_per_contact = lane_per_contact ? 1 : 0;
-    // speculative contacts live in the generic (CONVEX = true) instantiation only, with the two-kernel export
-    const bool generic = m->has_convex_pairs || M.spec_mode != 0 || m->has_mesh_pairs;  // mesh-plane pairs: generic instantiation only
-    const nb2_contacts_view* fused_out = (contacts && fused && M.spec_mode == 0) ? contacts : nullptr;
-#define NB2_COLLIDE_DISPATCH(LANES) \
-    st = generic ? launch_collide_L<LANES, true>(m, body_q, fused_out, s) : launch_collide_L<LANES, false>(m, body_q, fused_out, s)
+    // speculative contacts and mesh-plane pairs live in the generic (CONVEX = true) instantiation only
+    const bool generic = m->has_convex_pairs || M.spec_mode != 0 || m->has_mesh_pairs;
+#define COLLIDE_DISPATCH(LANES) st = generic ? launch_collide_L<LANES, true>(m, body_q, s) : launch_collide_L<LANES, false>(m, body_q, s)
     switch (m->lanes_per_env) {
-        case 8: NB2_COLLIDE_DISPATCH(8); break;
-        case 16: NB2_COLLIDE_DISPATCH(16); break;
-        default: NB2_COLLIDE_DISPATCH(32); break;
+        case 8: COLLIDE_DISPATCH(8); break;
+        case 16: COLLIDE_DISPATCH(16); break;
+        default: COLLIDE_DISPATCH(32); break;
     }
-#undef NB2_COLLIDE_DISPATCH
+#undef COLLIDE_DISPATCH
     if (st != NB2_OK) return st;
-    if (contacts && !fused_out) {
+    // The `Contacts` arrays are written by a second kernel.  Writing them from collide_kernel itself, with a decoupled look-back for
+    // the offsets, lost: 690.1 vs 678.3 us per 4096-quadruped frame (profiles/r2j_fused_export_ab.txt, DESIGN.md section 2).
+    if (contacts) {
         if (M.env_count <= 8192) {
             contact_export_kernel<true><<<(M.env_count + 3) / 4, 128, 0, s>>>(M, *contacts);
             count_launch();

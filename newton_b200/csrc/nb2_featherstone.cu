@@ -21,7 +21,6 @@
 // strict-fp build reproduces the CPU oracle bit for bit.  Tensor cores (north_star: "only for the small dense
 // mass-matrix factor/solve") would need TF32 or 3xTF32 splits and cannot meet bit-parity; with H at 18x18 the stage is
 // ~9 k MACs per env, latency- not throughput-bound, so it stays on the FP32 pipe (DESIGN.md §3).
-#include <cstdlib>
 
 #include "nb2_internal.cuh"
 #include "nb2_math.cuh"
@@ -397,17 +396,16 @@ __device__ __noinline__ void tile_mass_matrix(const float* S, const float* Is, c
 // profiles/r2b_xpbd_ab.txt).
 #define NB2_PHASE()                       \
     do {                                  \
-        if (WARPS > 1 && (kflags & 1)) __syncthreads(); \
+        if (WARPS > 1) __syncthreads();   \
     } while (0)
 template <int L, bool PF, int WARPS, bool TILE>
 __global__ void __launch_bounds__(32 * WARPS, (WARPS >= 14 ? 1 : 14 / WARPS))
 featherstone_step_kernel(DevModel M, nb2_featherstone_params P, nb2_state_view sin, nb2_state_view sout, nb2_control_view ctl, int use_contacts,
-                         int update_mass, float dt, int kflags) {  // kflags: 1 = CTA barrier at phase boundaries, 2 = shuffle-broadcast substitutions
+                         int update_mass, float dt) {
     constexpr int G = 32 / L;
     extern __shared__ float smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int grp = lane / L, l = lane % L;
-    if (int(blockIdx.x) * WARPS * G >= M.env_count) return;  // padding CTA of the NB2_FS_MIN_GRID experiment (before any barrier)
     const int env = (blockIdx.x * WARPS + warp) * G + grp;
     const bool live = env < M.env_count;
     // groups run different trip counts (articulations / dofs per env), so barriers cover one group only
@@ -957,63 +955,30 @@ featherstone_step_kernel(DevModel M, nb2_featherstone_params P, nb2_state_view s
         }
         __syncwarp(gmask);
         // dense_subs (kernels.py:1754-1781): forward then backward substitution, each row's subtractions in the serial loop's order
-        if (kflags & 2) {
-            // Row i belongs to lane i % L.  A finished unknown travels to the group by shuffle (no shared-memory round trip, no barrier
-            // per column); the lanes then update / prepare their own rows only, so every shared-memory cell is written and read by
-            // one thread.
+        {   // forward substitution, column-oriented: as soon as x[j] is final every later row subtracts L[i,j] x[j] - each row
+            // still performs its subtractions in ascending j and divides last, i.e. the serial loop's arithmetic
             float* x = sm.qdd + (ad0 - d0);
             const float* bvec = sm.tau + (ad0 - d0);
             for (int i = l; i < n; i += L) x[i] = bvec[i];
-            // forward, column-oriented: when x[j] is final every later row subtracts L[i,j] x[j] - ascending j per row, divide last
+            __syncwarp(gmask);
             for (int j = 0; j < n; ++j) {
-                const int owner = j % L;
-                float xj = 0.0f;
-                if (l == owner) {
-                    xj = x[j] / H[j * n + j];
-                    x[j] = xj;
-                }
-                xj = __shfl_sync(gmask, xj, owner, L);
-                for (int i = j + 1 + ((l - (j + 1)) % L + L) % L; i < n; i += L) x[i] -= H[i * n + j] * xj;
-            }
-            // backward: row i subtracts L[j,i] x[j] for j = i+1 .. n-1 in ascending j, i.e. it cannot start before x[i+1] - the LAST of
-            // them - is final.  The products do not have to wait: as soon as x[i] is final the lanes put L[i,r] x[i] for their rows
-            // r < i into the unused upper triangle (H[r, i]); the serial chain of row i is then one load and one subtraction per term.
-            for (int i = n - 1; i >= 0; --i) {
-                const int owner = i % L;
-                float xi = 0.0f;
-                if (l == owner) {
-                    float t = x[i];
-                    for (int j = i + 1; j < n; ++j) t -= H[i * n + j];
-                    xi = t / H[i * n + i];
-                    x[i] = xi;
-                }
-                xi = __shfl_sync(gmask, xi, owner, L);
-                for (int r = l; r < i; r += L) H[r * n + i] = H[i * n + r] * xi;
-            }
-        } else {
-            {   // forward substitution, column-oriented: as soon as x[j] is final every later row subtracts L[i,j] x[j] - each row
-                // still performs its subtractions in ascending j and divides last, i.e. the serial loop's arithmetic
-                float* x = sm.qdd + (ad0 - d0);
-                const float* bvec = sm.tau + (ad0 - d0);
-                for (int i = l; i < n; i += L) x[i] = bvec[i];
+                if (l == j % L) x[j] = x[j] / H[j * n + j];
                 __syncwarp(gmask);
-                for (int j = 0; j < n; ++j) {
-                    if (l == j % L) x[j] = x[j] / H[j * n + j];
-                    __syncwarp(gmask);
-                    const float xj = x[j];
-                    for (int i = j + 1 + ((l - (j + 1)) % L + L) % L; i < n; i += L) x[i] -= H[i * n + j] * xj;  // rows > j owned by this lane
-                }
-                __syncwarp(gmask);
-            }
-            if (l == 0) {  // backward substitution: every row needs ALL later unknowns before its first (ascending-order) subtraction
-                float* x = sm.qdd + (ad0 - d0);
-                for (int i = n - 1; i >= 0; --i) {
-                    float t = x[i];
-                    for (int j = i + 1; j < n; ++j) t -= H[j * n + i] * x[j];
-                    x[i] = t / H[i * n + i];
-                }
+                const float xj = x[j];
+                for (int i = j + 1 + ((l - (j + 1)) % L + L) % L; i < n; i += L) x[i] -= H[i * n + j] * xj;  // rows > j owned by this lane
             }
             __syncwarp(gmask);
+        }
+        // backward substitution: every row needs ALL later unknowns before its first (ascending-order) subtraction.  Shuffle-broadcast
+        // substitutions with the backward products staged in the upper triangle were bit-exact but slower: 82.4 vs 80.3 us at 4096
+        // quadruped envs (profiles/r2q_featherstone_subst_ab.txt)
+        if (l == 0) {
+            float* x = sm.qdd + (ad0 - d0);
+            for (int i = n - 1; i >= 0; --i) {
+                float t = x[i];
+                for (int j = i + 1; j < n; ++j) t -= H[j * n + i] * x[j];
+                x[i] = t / H[i * n + i];
+            }
         }
         __syncwarp(gmask);
         for (int i = l; i < n; i += L)  // zero_kinematic_joint_qdd (kernels.py:1933-1948)
@@ -1192,14 +1157,7 @@ static nb2_status launch_fs_W(nb2_model* m, const nb2_featherstone_params& p, co
     if (smem > 48 * 1024)
         NB2_CUDA_CHECK(cudaFuncSetAttribute(featherstone_step_kernel<L, PF, WARPS, TILE>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
     NB2_CUDA_CHECK(cudaFuncSetAttribute(featherstone_step_kernel<L, PF, WARPS, TILE>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    static const int phase_sync = std::getenv("NB2_FS_PHASE_SYNC") ? std::atoi(std::getenv("NB2_FS_PHASE_SYNC")) : 1;
-    // NB2_FS_SHFL_SUBST=1: substitutions with shuffle broadcasts and the products of the backward pass in the upper triangle.  Bit-exact
-    // (the round-2q GPU suite ran with it) but it LOSES: 82.4 vs 80.3 us at 4096 quadruped envs (profiles/r2q_featherstone_subst_ab.txt) -
-    // the divergent per-lane row loops around every shuffle cost more than the barriers they replace.  Default: the round-2p path.
-    static const int shfl_subst = std::getenv("NB2_FS_SHFL_SUBST") ? std::atoi(std::getenv("NB2_FS_SHFL_SUBST")) : 0;
-    const int kflags = (phase_sync ? 1 : 0) | (shfl_subst ? 2 : 0);
-    static const int min_grid = std::getenv("NB2_FS_MIN_GRID") ? std::atoi(std::getenv("NB2_FS_MIN_GRID")) : 0;  // A/B: idle padding CTAs
-    featherstone_step_kernel<L, PF, WARPS, TILE><<<blocks < min_grid ? min_grid : blocks, 32 * WARPS, smem, s>>>(M, p, in, out, ctl, use_contacts, update_mass, dt, kflags);
+    featherstone_step_kernel<L, PF, WARPS, TILE><<<blocks, 32 * WARPS, smem, s>>>(M, p, in, out, ctl, use_contacts, update_mass, dt);
     count_launch();
     NB2_CUDA_CHECK(cudaGetLastError());
     return NB2_OK;
@@ -1215,15 +1173,8 @@ static nb2_status launch_fs_LP(nb2_model* m, const nb2_featherstone_params& p, c
         set_error("featherstone_step: environment too large for the fused shared-memory kernel");
         return NB2_ERR_CAPACITY;
     }
-    static const int forced = std::getenv("NB2_FS_WARPS") ? std::atoi(std::getenv("NB2_FS_WARPS")) : 0;
-    int warps = forced;
-    if (warps <= 0) {
-        int sms = 148;
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, m->device);
-        const long long total_warps = (M.env_count + (32 / L) - 1) / (32 / L);
-        const long long per_sm = (total_warps + sms - 1) / sms;
-        warps = per_sm <= 1 ? 1 : (per_sm <= 4 ? 4 : 14);
-    }
+    const long long per_sm = warps_per_sm(m, L);
+    int warps = per_sm <= 1 ? 1 : (per_sm <= 4 ? 4 : 14);
     if (warps >= 14 && per_env * 14 > 220 * 1024) warps = 4;
     if (warps >= 4 && warps < 14 && per_env * 4 > 220 * 1024) warps = 1;
     if (p.use_tile_gemm) {

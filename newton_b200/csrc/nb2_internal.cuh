@@ -47,8 +47,6 @@ struct DevModel {
     int slot_total;
     int* env_contact_count;        // [E]
     int* env_contact_offset;       // [E+1] exclusive scan, written by the export path
-    int* collide_sync;             // [3] ticket / done / epoch of the fused export's tile chain (collide_kernel)
-    unsigned long long* collide_tile_status;  // [E] (epoch | flag | count) per tile: decoupled look-back of the export offsets
     int max_env_bodies, max_env_joints, max_env_slots_shapes, max_env_pairs, max_env_contact_slots;
     // articulated-body (Featherstone) tables
     const int* joint_depth;            // [J] depth of each joint in its articulation tree (root = 0)
@@ -83,7 +81,6 @@ struct DevModel {
     int filter_count;
     // speculative contacts (nb2_collide_speculative): 0 = off, 1 = enabled but inactive for this call (dt == 0 or extension == 0:
     // only the writer's admission rule changes), 2 = active (shape velocities, swept broad phase, velocity-extended search gaps)
-    int lane_per_contact;  // collide_kernel write-out: 1 = one lane per contact through a shared-memory staging area
     int spec_mode;
     int has_mesh_pairs;    // the explicit pair list holds (mesh, infinite plane) pairs
     const float* spec_body_qd;
@@ -113,6 +110,7 @@ struct HostTables {
 
 struct nb2_model {
     int device = 0;
+    int sm_count = 0;        // multiprocessors of `device`, queried at nb2_model_create
     nb2::DevModel dev{};
     nb2::HostTables host;
     std::vector<void*> allocations;
@@ -150,6 +148,12 @@ struct nb2_model {
 };
 
 namespace nb2 {
+// Warps per SM a launch with one environment per L-lane group needs to cover the batch in one wave.  The fused kernels' launchers
+// pick their CTA width from it.
+inline long long warps_per_sm(const nb2_model* m, int L) {
+    const long long total_warps = (m->dev.env_count + (32 / L) - 1) / (32 / L);
+    return (total_warps + m->sm_count - 1) / m->sm_count;
+}
 void set_error(const std::string& msg);
 void count_launch(int n = 1);
 nb2_status launch_collide(nb2_model* m, const float* body_q, const nb2_contacts_view* contacts, cudaStream_t s);

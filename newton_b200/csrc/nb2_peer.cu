@@ -9,7 +9,6 @@
 // Two receive slots (sequence parity) let frame f+1 land while frame f is still being read.
 #include <cuda.h>
 
-#include <cstdlib>
 #include <cstring>
 
 #include "nb2_internal.cuh"
@@ -22,9 +21,7 @@ struct nb2_peer_gather {
     std::vector<char*> peer_recv;  // peer-mapped addresses (own rank: the local pointers)
     std::vector<int*> peer_flags;
     int** d_peer_flags = nullptr;  // device copy of peer_flags for the signal kernel
-    bool memops = false;           // publish with cuStreamWriteValue32 instead of the one-thread signal kernel
     CUresult (*wait32)(CUstream, CUdeviceptr, cuuint32_t, unsigned int) = nullptr;
-    CUresult (*write32)(CUstream, CUdeviceptr, cuuint32_t, unsigned int) = nullptr;
 };
 
 namespace nb2 {
@@ -82,11 +79,7 @@ nb2_status nb2_peer_gather_create(int32_t device, int32_t rank, int32_t world_si
     void* fn = nullptr;
     if (cudaGetDriverEntryPoint("cuStreamWaitValue32", &fn, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
         g->wait32 = reinterpret_cast<decltype(g->wait32)>(fn);
-    fn = nullptr;
-    if (cudaGetDriverEntryPoint("cuStreamWriteValue32", &fn, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-        g->write32 = reinterpret_cast<decltype(g->write32)>(fn);
     cudaGetLastError();
-    if (const char* v = std::getenv("NB2_PEER_MEMOPS")) g->memops = std::atoi(v) != 0 && g->write32;
     if (prev >= 0 && prev != device) cudaSetDevice(prev);
     *out = g;
     return NB2_OK;
@@ -154,19 +147,11 @@ nb2_status nb2_peer_gather_push(nb2_peer_gather* g, const void* src, size_t byte
         }
         NB2_CUDA_CHECK(cudaMemcpyAsync(g->peer_recv[p] + slot_off, src, bytes, cudaMemcpyDefault, s));
     }
-    if (g->memops) {
-        for (int p = 0; p < g->world; ++p) {
-            const CUresult r = g->write32(s, reinterpret_cast<CUdeviceptr>(g->peer_flags[p] + flag_index), cuuint32_t(sequence), 0);
-            if (r != CUDA_SUCCESS) {
-                set_error("nb2_peer_gather_push: cuStreamWriteValue32 failed");
-                return NB2_ERR_CUDA;
-            }
-        }
-    } else {
-        peer_signal_kernel<<<1, 32, 0, s>>>(g->d_peer_flags, g->world, flag_index, sequence);
-        count_launch();
-        NB2_CUDA_CHECK(cudaGetLastError());
-    }
+    // The flag is published by a small kernel: publishing it with cuStreamWriteValue32 instead was not faster (0.7449 vs 0.7436 ms
+    // per frame at N = 2, DESIGN.md section 6).
+    peer_signal_kernel<<<1, 32, 0, s>>>(g->d_peer_flags, g->world, flag_index, sequence);
+    count_launch();
+    NB2_CUDA_CHECK(cudaGetLastError());
     return NB2_OK;
 }
 

@@ -15,8 +15,6 @@
 //     solve_body_joints             kernels.py:1513-2044  joint lanes -> smem delta records
 //     apply_body_deltas             kernels.py:864-933    body lanes, ordered sum over the body's joints (CSR)
 //   copy_kinematic_body_state      kernels.py:19-32       implicit: kinematic bodies are never modified
-#include <cstdlib>
-
 #include "nb2_internal.cuh"
 #include "nb2_math.cuh"
 
@@ -30,28 +28,13 @@ enum { BODY_KINEMATIC = 2 };
 // shared-memory body record (floats): odd stride -> consecutive bodies hit different banks
 enum { BR_Q = 0, BR_QD = 7, BR_COM = 13, BR_INVM = 16, BR_INVI = 17, BR_I = 26, BR_SIZE = 35 };
 enum { DR_SIZE = 13 };  // delta record: lin_a, ang_a, lin_b, ang_b, active
-enum { XF_JOINT_CACHE = 1, XF_TMA = 2, XF_PHASE_SYNC = 4, XF_PHASE_SYNC_FINE = 8 };  // kernel flags
 // per-contact constants of the Jacobi loop, staged once per substep: point0, point1, normal, margin0 + margin1, the three friction
 // coefficients and the friction anchors point + offset (odd stride: lanes = consecutive contacts)
 enum { CC_P0 = 0, CC_P1 = 3, CC_N = 6, CC_MSUM = 9, CC_MU = 10, CC_MUT = 11, CC_MUR = 12, CC_Q0 = 13, CC_Q1 = 16, CC_SIZE = 19 };
 
-// Code-size control.  The first kernel version inlined and unrolled everything: 9 400 SASS instructions (150 KB) and
-// 19 % of the stall samples on instruction fetch (profiles/r1a_xpbd_step_kernel.txt).  With one-warp CTAs (round 1) rolled vs.
-// unrolled 3-row joint loops and real calls vs. inlined helpers all timed within 1 % of each other
-// (profiles/r1c_xpbd_code_size_ab.txt).  With 14-warp CTAs walking the code together (round 2) the instruction stream is fetched once
-// per CTA, and the unrolled rows win: no per-row component selects / loop control, three independent rows for the scheduler to
-// interleave - 143.7 -> 139.7 us at 4096 quadruped envs (profiles/r2j_fused_export_ab.txt), so unrolled is the default.
-// -DNB2_XPBD_ROLLED / -DNB2_XPBD_NOINLINE rebuild the other variants.
-#ifdef NB2_XPBD_NOINLINE
-#define NB2_HELPER __host__ __device__ __noinline__
-#else
-#define NB2_HELPER NB2_DEV
-#endif
-#ifndef NB2_XPBD_ROLLED
-#define NB2_ROW_UNROLL _Pragma("unroll")
-#else
-#define NB2_ROW_UNROLL _Pragma("unroll 1")
-#endif
+// Code size.  With 14-warp CTAs walking the code together the instruction stream is fetched once per CTA, so the helpers are inlined
+// and the 3-row joint loops unrolled: no per-row component selects / loop control, three independent rows for the scheduler to
+// interleave.  Unrolled rows: 143.7 -> 139.7 us at 4096 quadruped envs (profiles/r2j_fused_export_ab.txt).
 
 struct BodyView {
     Xf X;
@@ -80,7 +63,7 @@ NB2_DEV BodyView static_body() {  // body index -1: the world
 
 // r^T I^-1 r with r = ang rotated into the body frame: the angular term of the generalized inverse mass.  For the static
 // world the reference multiplies by a zero inverse inertia; the sum is +-0 and adding it leaves the denominator unchanged.
-NB2_HELPER float ang_inv_mass(const float* rec, V3 ang) {
+NB2_DEV float ang_inv_mass(const float* rec, V3 ang) {
     if (rec == nullptr) return 0.0f;
     const Q4 q(rec[BR_Q + 3], rec[BR_Q + 4], rec[BR_Q + 5], rec[BR_Q + 6]);
     const V3 r = qrot_inv(q, ang);
@@ -271,7 +254,7 @@ NB2_DEV bool solve_joint(const nb2_model_desc& d, const nb2_control_view& ctl, c
         }
         const V3 r_p = xpoint(X_wp, proj) - wcom_p;
         const V3 r_c = x_c - wcom_c;
-        NB2_ROW_UNROLL
+#pragma unroll
         for (int dim = 0; dim < 3; ++dim) {
             float e = rel_p.get(dim);
             // column `dim` of quat_to_matrix(X_wp.q), i.e. the rotated basis vector
@@ -334,7 +317,7 @@ NB2_DEV bool solve_joint(const nb2_model_desc& d, const nb2_control_view& ctl, c
         }
         const AxisSetup s = jc ? load_axis_setup(jc + JC_ANG) : gather_axes(d, ctl, axis_start, target_start, lin_count, ang_count);
         const Q4 qc_inv = qconj(q_c);
-        NB2_ROW_UNROLL
+#pragma unroll
         for (int dim = 0; dim < 3; ++dim) {
             float e = dim == 0 ? err_0 : (dim == 1 ? err_1 : err_2);
             Q4 grad = dim == 0 ? g0 : (dim == 1 ? g1 : g2);
@@ -432,7 +415,7 @@ NB2_DEV void store_deltas(float* rec, const Deltas& dl, float active) {
 }
 
 // apply_body_deltas for one body held in shared memory (kernels.py:864-933), in place.
-NB2_HELPER void apply_delta(float* rec, V3 dlin, V3 dang, float inv_weight, bool weighted, float dt) {
+NB2_DEV void apply_delta(float* rec, V3 dlin, V3 dang, float inv_weight, bool weighted, float dt) {
     const float inv_m = rec[BR_INVM];
     if (inv_m == 0.0f) return;
     const M33 inv_I = ldm(rec + BR_INVI), I = ldm(rec + BR_I);
@@ -526,18 +509,15 @@ enum { ST_Q = 0, ST_QD = 7, ST_COM = 13, ST_INVM = 16, ST_I = 17, ST_INVI = 26, 
 // WARPS warps per CTA, each warp = 32/L environments.  All warps of a CTA walk the same code at about the same time, so the
 // 6 500-instruction iteration body (far larger than the 32 KB L1.5 instruction cache) is fetched once per CTA instead of once per
 // warp; one-warp CTAs each at their own PC were 18 % `stall_no_inst` (profiles/r1f_xpbd_step_kernel.txt).
-#ifndef NB2_XPBD_MIN_WARPS
-#define NB2_XPBD_MIN_WARPS 16  // resident warps per SM the register allocation must allow (16 -> 128 registers)
-#endif
+constexpr int XPBD_MIN_WARPS = 16;  // resident warps per SM the register allocation must allow (16 -> 128 registers)
 template <int L, bool EX, int WARPS>
-__global__ void __launch_bounds__(32 * WARPS, (WARPS >= NB2_XPBD_MIN_WARPS ? 1 : NB2_XPBD_MIN_WARPS / WARPS))
+__global__ void __launch_bounds__(32 * WARPS, (WARPS >= XPBD_MIN_WARPS ? 1 : XPBD_MIN_WARPS / WARPS))
 xpbd_step_kernel(DevModel M, nb2_xpbd_params P, nb2_state_view sin, nb2_state_view sout, nb2_control_view ctl, int use_contacts_flags,
-                 float dt, int flags, int contact_cap, int contact_cache) {
+                 float dt, bool joint_cache, int contact_cap, int contact_cache) {
     const int use_contacts = use_contacts_flags & NB2_XPBD_USE_CONTACTS;
     const bool want_cimp = EX && use_contacts && (use_contacts_flags & NB2_XPBD_CONTACT_IMPULSE);
     const bool want_jimp = EX && sout.body_parent_f != nullptr;
     const bool want_init = EX && (P.enable_restitution || P.compute_body_velocity_from_position_delta);
-    const bool joint_cache = (flags & XF_JOINT_CACHE) != 0;
     constexpr int G = 32 / L;
     constexpr int NE = G * WARPS;
     extern __shared__ __align__(16) float smem[];
@@ -545,7 +525,6 @@ xpbd_step_kernel(DevModel M, nb2_xpbd_params P, nb2_state_view sin, nb2_state_vi
     const int grp = lane / L, l = lane % L;
     const int slot = warp * G + grp;  // environment slot inside the CTA
     const int env0 = blockIdx.x * NE;
-    if (env0 >= M.env_count) return;  // padding CTA of the NB2_XPBD_MIN_GRID experiment (whole CTA, before any barrier)
     const int env = env0 + slot;
     const bool live = env < M.env_count;
     const nb2_model_desc& d = M.d;
@@ -573,7 +552,7 @@ xpbd_step_kernel(DevModel M, nb2_xpbd_params P, nb2_state_view sin, nb2_state_vi
     // CTA-uniform decision: the CTA's body run [cb0, cb0 + cnb) must be 16-byte aligned in every array it is copied from / to
     const int env_last = min(env0 + NE, M.env_count);
     const int cb0 = M.env_body_start[env0], cnb = M.env_body_start[env_last] - cb0;
-    bool tma = (flags & XF_TMA) != 0 && cnb > 0 && (cb0 & 3) == 0 && (cnb & 3) == 0 && cnb * ST_PER_BODY <= NE * plan.rec_cap * DR_SIZE;
+    bool tma = cnb > 0 && (cb0 & 3) == 0 && (cnb & 3) == 0 && cnb * ST_PER_BODY <= NE * plan.rec_cap * DR_SIZE;
     if (tma) {
         const uintptr_t a = reinterpret_cast<uintptr_t>(sin.body_q) | reinterpret_cast<uintptr_t>(sin.body_qd) |
                             reinterpret_cast<uintptr_t>(sout.body_q) | reinterpret_cast<uintptr_t>(sout.body_qd) |
@@ -751,9 +730,9 @@ xpbd_step_kernel(DevModel M, nb2_xpbd_params P, nb2_state_view sin, nb2_state_vi
     const float lin_alpha_dt = P.joint_linear_compliance / dt, ang_alpha_dt = P.joint_angular_compliance / dt;
     for (int it = 0; it < P.iterations; ++it) {
         // CTA barriers are not needed for correctness (a warp owns its environments); they keep the CTA's warps on the same
-        // stretch of code so that the instruction stream is fetched once per CTA (see the kernel comment)
-        const bool sync_it = (flags & XF_PHASE_SYNC) && WARPS > 1, sync_fine = (flags & XF_PHASE_SYNC_FINE) && WARPS > 1;
-        if (sync_it) __syncthreads();
+        // stretch of code so that the instruction stream is fetched once per CTA (see the kernel comment).  One per iteration: 147.8 us,
+        // against 154.4 us without barriers and 151.9 us with one at every phase boundary (DESIGN.md section 3.1)
+        if (WARPS > 1) __syncthreads();
         if (use_contacts) {
             // ---- [iteration] solve_body_contact_positions (kernels.py:2164-2399)
             for (int c = l; c < nc; c += L) {
@@ -854,7 +833,6 @@ xpbd_step_kernel(DevModel M, nb2_xpbd_params P, nb2_state_view sin, nb2_state_vi
                 store_deltas(drec + c * DR_SIZE, dl, active);
             }
             __syncwarp();
-            if (sync_fine) __syncthreads();
             // ---- [iteration] ordered per-body sum (contact order; side A before side B) + weighted apply
             for (int b = l; b < nb; b += L) {
                 V3 dlin, dang;
@@ -908,7 +886,6 @@ xpbd_step_kernel(DevModel M, nb2_xpbd_params P, nb2_state_view sin, nb2_state_vi
             }
         }
         if (d.joint_count > 0) {
-            if (sync_fine) __syncthreads();
             // ---- [iteration] solve_body_joints (kernels.py:1513-2044) + ordered per-body apply
             for (int j = l; j < nj; j += L) {
                 Deltas dl;
@@ -923,7 +900,6 @@ xpbd_step_kernel(DevModel M, nb2_xpbd_params P, nb2_state_view sin, nb2_state_vi
                 }
             }
             __syncwarp();
-            if (sync_fine) __syncthreads();
             for (int b = l; b < nb; b += L) {
                 const int gb = b0 + b;
                 V3 dlin, dang;
@@ -1144,11 +1120,6 @@ __global__ void __launch_bounds__(256) integrate_bodies_kernel(nb2_model_desc d,
     st3(sout.body_qd + 6 * b + 3, w1);
 }
 
-static int env_int(const char* name, int fallback) {
-    const char* v = std::getenv(name);
-    return v ? std::atoi(v) : fallback;
-}
-
 template <int L, bool EX, int WARPS>
 static nb2_status launch_xpbd_W(nb2_model* m, const nb2_xpbd_params& p, const nb2_state_view& in, const nb2_state_view& out,
                                 const nb2_control_view& ctl, int use_contacts, float dt, cudaStream_t s) {
@@ -1164,31 +1135,28 @@ static nb2_status launch_xpbd_W(nb2_model* m, const nb2_xpbd_params& p, const nb
     }
     // Budget: the CTAs of one SM share 227 KB (+1 KB reserved each); the batch wants >= ceil(envs / (G * 148)) resident warps per SM to
     // stay a single wave.  The per-joint cache rides along when it does not cost that residency.
-    static const bool cache_enabled = std::getenv("NB2_XPBD_NO_JOINT_CACHE") == nullptr;  // A/B switch (profiles/r1f_xpbd_ab.txt)
-    static const int tma_enabled = env_int("NB2_XPBD_TMA", 1), phase_sync = env_int("NB2_XPBD_PHASE_SYNC", 1);
-    int flags = (tma_enabled ? XF_TMA : 0) | (phase_sync >= 1 ? XF_PHASE_SYNC : 0) | (phase_sync >= 2 ? XF_PHASE_SYNC_FINE : 0);
+    bool joint_cache = false;
     XpbdPlan plan = xpbd_plan(NE, M.max_env_bodies, M.max_env_joints, contact_cap, EX, false);
-    if (cache_enabled && M.d.joint_count > 0) {
+    if (M.d.joint_count > 0) {
         const XpbdPlan with_cache = xpbd_plan(NE, M.max_env_bodies, M.max_env_joints, contact_cap, EX, true);
         const int want_ctas = (14 + WARPS - 1) / WARPS;  // 14 warps per SM keep 4096 two-env warps in one wave
         if ((size_t(with_cache.total) * sizeof(float) + 1024) * want_ctas <= 227 * 1024 || size_t(plan.total) * sizeof(float) * want_ctas > 227 * 1024) {
             if (size_t(with_cache.total) * sizeof(float) <= 220 * 1024) {
                 plan = with_cache;
-                flags |= XF_JOINT_CACHE;
+                joint_cache = true;
             }
         }
     }
     // contact-constant cache: as many contacts per env as still fit (up to the contact bound), keeping the residency above
     int contact_cache = 0;
     {
-        static const int cc_enabled = env_int("NB2_XPBD_CONTACT_CACHE", 1);
         const int want_ctas = (14 + WARPS - 1) / WARPS;
         const size_t budget = (size_t(227) * 1024) / want_ctas - 1024 - 64;
         const size_t base = size_t(plan.total) * sizeof(float);
-        if (cc_enabled && use_contacts && base < budget) {
+        if (use_contacts && base < budget) {
             contact_cache = int(std::min<size_t>((budget - base) / (size_t(NE) * CC_SIZE * sizeof(float)), size_t(contact_cap)));
             if (contact_cache > 0)
-                plan = xpbd_plan(NE, M.max_env_bodies, M.max_env_joints, contact_cap, EX, (flags & XF_JOINT_CACHE) != 0, contact_cache);
+                plan = xpbd_plan(NE, M.max_env_bodies, M.max_env_joints, contact_cap, EX, joint_cache, contact_cache);
         }
     }
     const size_t smem = size_t(plan.total) * sizeof(float);
@@ -1199,12 +1167,8 @@ static nb2_status launch_xpbd_W(nb2_model* m, const nb2_xpbd_params& p, const nb
     if (smem > 48 * 1024)
         NB2_CUDA_CHECK(cudaFuncSetAttribute(xpbd_step_kernel<L, EX, WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
     // ask for the largest shared-memory carve-out so that ~14-16 warps' worth of CTAs fit per SM
-    static const int carveout = std::getenv("NB2_XPBD_CARVEOUT") ? std::atoi(std::getenv("NB2_XPBD_CARVEOUT")) : int(cudaSharedmemCarveoutMaxShared);
-    NB2_CUDA_CHECK(cudaFuncSetAttribute(xpbd_step_kernel<L, EX, WARPS>, cudaFuncAttributePreferredSharedMemoryCarveout, carveout));
-    // A/B switch: pad the grid with idle CTAs up to this many (profiles/: does a grid below the SM count change the issue rate?)
-    static const int min_grid = env_int("NB2_XPBD_MIN_GRID", 0);
-    const int grid = blocks < min_grid ? min_grid : blocks;
-    xpbd_step_kernel<L, EX, WARPS><<<grid, 32 * WARPS, smem, s>>>(M, p, in, out, ctl, use_contacts, dt, flags, contact_cap, contact_cache);
+    NB2_CUDA_CHECK(cudaFuncSetAttribute(xpbd_step_kernel<L, EX, WARPS>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    xpbd_step_kernel<L, EX, WARPS><<<blocks, 32 * WARPS, smem, s>>>(M, p, in, out, ctl, use_contacts, dt, joint_cache, contact_cap, contact_cache);
     count_launch();
     NB2_CUDA_CHECK(cudaGetLastError());
     return NB2_OK;
@@ -1213,19 +1177,12 @@ static nb2_status launch_xpbd_W(nb2_model* m, const nb2_xpbd_params& p, const nb
 // Warps per CTA.  Measured on B200 (profiles/r2b_xpbd_ab.txt, 4096 quadruped envs): 1 / 2 / 4 warps 166 us, 7 warps 160 us,
 // 14 warps 155 us, and 148 us with the per-iteration CTA barrier - the more warps walk the same code together, the fewer times the
 // instruction stream is fetched.  The launch takes the largest compiled width that the batch can fill on every SM
-// (14 = one CTA per SM for 4096 two-env warps), falls back when shared memory does not allow it, and honours NB2_XPBD_WARPS.
+// (14 = one CTA per SM for 4096 two-env warps) and falls back when shared memory does not allow it.
 template <int L, bool EX>
 static nb2_status launch_xpbd_L(nb2_model* m, const nb2_xpbd_params& p, const nb2_state_view& in, const nb2_state_view& out,
                                 const nb2_control_view& ctl, int use_contacts, float dt, cudaStream_t s) {
-    static const int forced = env_int("NB2_XPBD_WARPS", 0);
-    int warps = forced;
-    if (warps <= 0) {
-        int sms = 148;
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, m->device);
-        const long long total_warps = (m->dev.env_count + (32 / L) - 1) / (32 / L);
-        const long long per_sm = (total_warps + sms - 1) / sms;
-        warps = per_sm <= 1 ? 1 : (per_sm <= 4 ? 4 : 14);
-    }
+    const long long per_sm = warps_per_sm(m, L);
+    int warps = per_sm <= 1 ? 1 : (per_sm <= 4 ? 4 : 14);
     // shared-memory fit (the per-CTA plan grows with the warp count)
     auto fits = [&](int w) {
         const int ne = (32 / L) * w;
@@ -1234,12 +1191,6 @@ static nb2_status launch_xpbd_L(nb2_model* m, const nb2_xpbd_params& p, const nb
     };
     if (warps >= 14 && !fits(14)) warps = 4;
     if (warps >= 4 && warps < 14 && !fits(4)) warps = 1;
-#ifdef NB2_XPBD_AB_VARIANTS
-    if constexpr (L == 16 && !EX) {
-        if (warps == 2) return launch_xpbd_W<L, EX, 2>(m, p, in, out, ctl, use_contacts, dt, s);
-        if (warps == 7) return launch_xpbd_W<L, EX, 7>(m, p, in, out, ctl, use_contacts, dt, s);
-    }
-#endif
     if (warps >= 14) return launch_xpbd_W<L, EX, 14>(m, p, in, out, ctl, use_contacts, dt, s);
     if (warps >= 4) return launch_xpbd_W<L, EX, 4>(m, p, in, out, ctl, use_contacts, dt, s);
     return launch_xpbd_W<L, EX, 1>(m, p, in, out, ctl, use_contacts, dt, s);
@@ -1263,15 +1214,15 @@ nb2_status launch_xpbd_step(nb2_model* m, const nb2_xpbd_params& p, const nb2_st
     }
     const bool ex = p.enable_restitution || p.compute_body_velocity_from_position_delta || out.body_parent_f != nullptr ||
                     ((use_contacts & NB2_XPBD_CONTACT_IMPULSE) && (use_contacts & NB2_XPBD_USE_CONTACTS));
-#define NB2_XPBD_DISPATCH(LANES)                                                                        \
+#define XPBD_DISPATCH(LANES)                                                                        \
     return ex ? launch_xpbd_L<LANES, true>(m, p, in, out, ctl, use_contacts, dt, s)                     \
               : launch_xpbd_L<LANES, false>(m, p, in, out, ctl, use_contacts, dt, s)
     switch (m->lanes_per_env) {
-        case 8: NB2_XPBD_DISPATCH(8);
-        case 16: NB2_XPBD_DISPATCH(16);
-        default: NB2_XPBD_DISPATCH(32);
+        case 8: XPBD_DISPATCH(8);
+        case 16: XPBD_DISPATCH(16);
+        default: XPBD_DISPATCH(32);
     }
-#undef NB2_XPBD_DISPATCH
+#undef XPBD_DISPATCH
 }
 
 nb2_status launch_xpbd_update_contacts(nb2_model* m, const nb2_contacts_view& contacts, cudaStream_t s) {

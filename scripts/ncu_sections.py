@@ -8,7 +8,7 @@ raw = subprocess.run(["ncu", "-i", rep, "--page", "source", "--csv", "--print-so
 rows = list(csv.reader(raw.splitlines()))
 lines = open(cu).read().splitlines()
 marks = [(i + 1, l.strip()[:90]) for i, l in enumerate(lines)
-         if re.match(r"\s*// ----", l) or re.match(r"^(NB2_DEV|NB2_HELPER|NB2_CALL|__global__|static|template)\b.*\(", l)]
+         if re.match(r"\s*// ----", l) or re.match(r"^(NB2_DEV|NB2_CALL|__global__|static|template)\b.*\(", l)]
 def section(ln):
     name = "(before first section)"
     for m, t in marks:
